@@ -46,6 +46,10 @@ TRAFFIC_FILE = os.path.join(ROOT, "profiles", "traffic.json")
 ALG_BYTES_PER_SAMPLE = 12  # dominant kernel, SURVEY §8d: read IQ 8 B + write qad 4 B (pulse table ~0.1 B/sample ignored)
 STEP_BYTES_PER_SAMPLE = {"detect": 16, "given": 12}  # SURVEY §8d per-path budgets (detect: qad re-read once)
 PARITY_LOG2 = 24  # parity windows of 2^24 samples (first / middle / last of every shard)
+# --dump-outputs: at most this many demodulated samples and pulse-table rows over all ranks, at fixed seeded positions when the
+# output is larger (qad 12 B per sample with its index, rows 24 B: 48 MB in all)
+DUMP_QAD_SAMPLES = 1 << 21
+DUMP_PULSE_ROWS = 1 << 20
 
 
 def env_int(name, default):
@@ -136,9 +140,10 @@ def _reference_detect_center():
         return oracle.detect_center, "port"
 
 
-def cpu_reference_arm(n_cpu, steps, warmup, iq_slice=None, detect=True):
-    """Time the reference's own CPU implementation (oracle/_ref compiled from /root/reference if it travelled
-    here, else the C oracle port) of afp_demod(FSK) [+ detect_center] + grab_pulse_lens on a bounded slice, all host threads."""
+def cpu_reference_arm(n_cpu, steps, warmup, iq_slice=None, detect=True, outputs=None):
+    """Time the reference's own CPU implementation (its compiled kernels under oracle/_ref when present, else the C oracle
+    port) of afp_demod(FSK) [+ detect_center] + grab_pulse_lens on a bounded slice, all host threads.  `outputs` (a dict)
+    receives the last step's qad, center and pulse table."""
     from oracle import oracle, ref_loader
 
     cores = os.cpu_count() or 1
@@ -171,6 +176,8 @@ def cpu_reference_arm(n_cpu, steps, warmup, iq_slice=None, detect=True):
         if it >= warmup:
             times.append(dt)
     sec = float(np.median(times))
+    if outputs is not None:
+        outputs.update(qad=q, center=center, rows=rows)
     return {"value": n_cpu / sec / 1e6, "unit": "MSamples/s", "cores": cores, "kind": kind,
             "sample": "%d-sample slice of the same synthetic 2-FSK recipe (afp_demod FSK [%s]%s + grab_pulse_lens [%s]), median of %d"
                       % (n_cpu, kind, (" + detect_center [%s, numpy as in the reference]" % center_kind) if detect else "", kind, len(times)),
@@ -191,6 +198,33 @@ def host_synth(n, seed=0):
     iq[:, 0] = x.real
     iq[:, 1] = x.imag
     return iq
+
+
+def dump_outputs(dirname, rank, world, n, get_qad, rows, center):
+    """Write what the step hands its caller - the detected (or given) center, the pulse table and the demodulated signal (qad) -
+    as float64 / float32 .npy files under `dirname` (suffix _rank<r> when world > 1).  Tables larger than the dump budget are
+    sampled at positions drawn with a fixed seed, so two builds run with the same arguments write comparable files; the *_index
+    files hold the positions.  get_qad(a, b) returns qad[a:b] on the host."""
+    os.makedirs(dirname, exist_ok=True)
+    sfx = "" if world == 1 else "_rank%d" % rank
+    rng = np.random.default_rng(20240 + rank)
+
+    def positions(total, cap):
+        return np.arange(total) if total <= cap else np.unique(rng.integers(0, total, cap))
+
+    qi = positions(n, DUMP_QAD_SAMPLES // world)
+    qad = np.empty(len(qi), np.float32)
+    chunk = 1 << 26
+    for a in range(0, n, chunk):
+        lo, hi = np.searchsorted(qi, [a, min(a + chunk, n)])
+        if hi > lo:
+            qad[lo:hi] = get_qad(a, min(a + chunk, n))[qi[lo:hi] - a]
+    ri = positions(len(rows), DUMP_PULSE_ROWS // world)
+    out = {"center": np.array([np.nan if center is None else center], np.float64),
+           "qad": qad, "qad_index": qi.astype(np.float64),
+           "pulses": rows[ri].astype(np.float64), "pulses_index": ri.astype(np.float64)}
+    for name, arr in out.items():
+        np.save(os.path.join(dirname, name + sfx + ".npy"), arr)
 
 
 def parity_windows(n_local):
@@ -285,10 +319,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the last step's center, pulse table and qad (sampled) to DIR/<name>.npy")
     ap.add_argument("--worst", action="store_true",
                     help="also time the unfavourable inputs (noise gate off / white-noise IQ / +-300 kHz deviation: every sample pair "
                          "leaves the packed-f32x2 fast path) and report them under `worst_case`")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = env_int("RANK", 0)
     local_rank = env_int("LOCAL_RANK", 0)
@@ -308,7 +346,10 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        r = cpu_reference_arm(1 << args.cpu_log2n, 5, max(1, min(args.warmup, 2)), detect=args.center == "detect")
+        last = {}
+        r = cpu_reference_arm(1 << args.cpu_log2n, args.steps, max(1, min(args.warmup, 2)), detect=args.center == "detect", outputs=last)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, 0, 1, len(last["qad"]), lambda a, b: last["qad"][a:b], last["rows"], last["center"])
         line = dict(base)
         line.update({"impl": "reference", "value": r["value"], "ms_per_step": r["ms_per_step"],
                      "cpu_baseline": {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")},
@@ -428,12 +469,17 @@ def main():
     ms_per_step = total_ms / args.steps
     value = world * n / (ms_per_step * 1e-3) / 1e6
 
-    # ---- parity of the last timed step against the CPU oracle (outside the timed region) ----------------------------
-    parity = None
-    if not args.no_parity:
+    # ---- the last timed step's outputs, and their parity against the CPU oracle (outside the timed region) -----------
+    rows_last = None
+    if args.dump_outputs or not args.no_parity:
         rows_last = np.empty((k_rows, 2), dtype=np.int64)
         if k_rows:
             ctx.check(lib.urh_fetch_pulses(ctx.handle, rows_last.ctypes.data_as(C.c_void_p), k_rows))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, n, lambda a, b: d_qad[a:b].get(), rows_last,
+                     center_seen[0] if args.center == "detect" else CENTER)
+    parity = None
+    if not args.no_parity:
         lens = int(rows_last[:, 1].sum())
         if dist is not None:
             import torch

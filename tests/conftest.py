@@ -1,3 +1,4 @@
+import hashlib
 import json
 import os
 import sys
@@ -25,6 +26,66 @@ def load_golden(name):
 
 
 CAPTURES = ["fsk", "ask", "ask_short", "psk_gen_noisy", "enocean", "FSK10", "homematic", "esaver", "two_participants"]
+
+# What the original project returned in the parity tests, one digest per case (tests/golden/make_golden_parity.py)
+REFERENCE_PARITY = os.path.join(GOLDEN, "reference_parity.json")
+
+
+def _feed(h, x):
+    if isinstance(x, dict):
+        h.update(b"{%d" % len(x))
+        for k in sorted(x, key=repr):
+            _feed(h, k)
+            _feed(h, x[k])
+        return
+    if isinstance(x, type):
+        x = np.dtype(x) if issubclass(x, np.generic) else x.__name__   # np.float32 == np.dtype("float32")
+    if x is None or isinstance(x, (str, bytes, np.dtype)):
+        s = x if isinstance(x, bytes) else repr(str(x) if isinstance(x, np.dtype) else x).encode()
+        h.update(b"s%d:" % len(s) + s)
+        return
+    scalar = (int, float, bool, np.number, np.bool_)
+    if isinstance(x, (list, tuple)) and not all(isinstance(v, scalar) for v in x):
+        h.update(b"[%d" % len(x))
+        for v in x:
+            _feed(h, v)
+        return
+    a = np.asarray(x)
+    if a.dtype == object or a.ndim > 1:
+        _feed(h, list(a))
+        return
+    if a.dtype.kind == "c":
+        h.update(b"c")
+        _feed(h, a.real)
+        a = a.imag
+    h.update(b"n" if a.ndim == 0 else b"v%d" % a.size)
+    if a.dtype.kind == "f":
+        a = a.astype(np.float64) + 0.0                              # -0.0 == 0.0
+        if np.all(np.isfinite(a)) and np.all(a == np.round(a)) and np.all(np.abs(a) < 2.0 ** 62):
+            a = a.astype(np.int64)                                  # 3.0 == 3
+    if a.dtype.kind == "f":
+        h.update(b"f" + np.where(np.isnan(a), np.nan, a).tobytes())
+    else:
+        h.update(b"i" + a.astype(np.int64).tobytes())
+
+
+def fingerprint(obj) -> str:
+    """Digest of a value as `==` / np.array_equal compare it: numbers by value (1 == 1.0 == np.int64(1)), lists, tuples and
+    arrays element by element, dicts by sorted items; strings, bytes and dtypes exactly.  To compare bit patterns and dtypes,
+    pass (a.dtype, a.shape, a.tobytes())."""
+    h = hashlib.sha256()
+    _feed(h, obj)
+    return h.hexdigest()[:16]
+
+
+def assert_matches_reference(key, observations):
+    """observations[i] (any value fingerprint() takes) equals what the original project gave for case i"""
+    with open(REFERENCE_PARITY) as f:
+        want = json.load(f)[key]
+    got = [fingerprint(o) for o in observations]
+    assert len(got) == len(want), (key, len(got), len(want))
+    bad = [i for i, (g, w) in enumerate(zip(got, want)) if g != w]
+    assert not bad, "%s: cases %s differ from the original project" % (key, bad[:20])
 
 
 @pytest.fixture(scope="session")

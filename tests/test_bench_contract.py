@@ -5,14 +5,10 @@ import os
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_reference_arm_line():
-    if not os.path.isdir(os.path.join(ROOT, "oracle", "_ref")) and not os.path.isdir("/root/reference"):
-        pytest.skip("no compiled reference and no reference tree")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
                           "--cpu-log2n", "18"], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
@@ -26,6 +22,24 @@ def test_reference_arm_line():
     e = d["e2e"]
     assert e["value"] == d["value"] and e["unit"] == d["unit"] and e["h2d_bytes_per_step"] == 0 and e["d2h_bytes_per_step"] == 0
     assert d["config"]["workload"].startswith("2-FSK complex64")
+
+
+def test_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs: the last step's center, pulse table and qad as float .npy files, the same from run to run"""
+    import numpy as np
+
+    runs = []
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1",
+                              "--cpu-log2n", "16", "--dump-outputs", str(tmp_path / d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        runs.append({f[:-4]: np.load(str(tmp_path / d / f)) for f in os.listdir(str(tmp_path / d))})
+    a, b = runs
+    assert sorted(a) == ["center", "pulses", "pulses_index", "qad", "qad_index"] == sorted(b)
+    for f in a:
+        assert a[f].dtype in (np.float32, np.float64) and np.array_equal(a[f], b[f]), f
+    assert len(a["qad"]) == 1 << 16 and np.array_equal(a["qad_index"], np.arange(1 << 16))
+    assert a["pulses"][:, 1].sum() == (1 << 16) - 5                      # every sample but the tolerance lies in some pulse
 
 
 def test_reference_arm_other_ranks_exit_quietly():

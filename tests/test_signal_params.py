@@ -1,13 +1,10 @@
-"""CPU: the parameter setters of urh_b200.signalprocessing.Signal (one descriptor table) behave like the reference's
+"""CPU: the parameter setters of urh_b200.signalprocessing.Signal (one descriptor table) behave like the original project's
 hand-written properties (Signal.py:215-400): same values, same events in the same order with the same arguments, same
-invalidation of the cached demodulation.  Needs the reference tree (build container); skipped elsewhere."""
-import os
-
+invalidation of the cached demodulation.  The observe_* functions run the cases on a Signal class; the tests compare this
+project's results with the digests tests/golden/make_golden_parity.py stored from the original's Signal."""
 import numpy as np
-import pytest
 
-REF = "/root/reference/src/urh/signalprocessing/Signal.py"
-pytestmark = pytest.mark.skipif(not os.path.isfile(REF), reason="reference tree not present")
+from conftest import assert_matches_reference
 
 EVENTS = ("samples_per_symbol_changed", "tolerance_changed", "noise_threshold_changed", "center_changed",
           "center_spacing_changed", "name_changed", "sample_rate_changed", "modulation_type_changed",
@@ -49,69 +46,74 @@ SCRIPT = [
 ]
 
 
-def test_parameter_setters_match_reference():
-    from oracle import ref_loader
-    ns = ref_loader.load_python_layer()
-    from urh_b200.signalprocessing.Signal import Signal
-
-    mine, ref = Signal("", "x", sample_rate=1e6), ns.Signal("", "x", sample_rate=1e6)
-    log_mine, log_ref = instrument(mine), instrument(ref)
+def observe_parameter_setters(Signal):
+    sig = Signal("", "x", sample_rate=1e6)
+    log = instrument(sig)
+    out = []
     for attr, value in SCRIPT:
-        for s in (mine, ref):
-            s._qad = np.zeros(3, np.float32)   # a cached demodulation that the setter may have to drop
-        setattr(mine, attr, value)
-        setattr(ref, attr, value)
-        assert (mine._qad is None) == (ref._qad is None), (attr, value)
+        sig._qad = np.zeros(3, np.float32)   # a cached demodulation that the setter may have to drop
+        setattr(sig, attr, value)
+        rec = [sig._qad is None]
         if attr != "block_protocol_update":
-            assert getattr(mine, attr) == getattr(ref, attr), (attr, value)
-            assert type(getattr(mine, attr)) is type(getattr(ref, attr)), (attr, value)
-    assert log_mine == log_ref
-    assert mine.modulation_order == ref.modulation_order == 8
+            v = getattr(sig, attr)
+            rec += [v, type(v).__name__]
+        out.append(rec)
+    out.append(log)
+    out.append(sig.modulation_order)
+    return out
 
 
-def test_construction_defaults_match_reference():
-    from oracle import ref_loader
-    ns = ref_loader.load_python_layer()
-    from urh_b200.signalprocessing.Signal import Signal
-
+def observe_construction_defaults(Signal):
+    out = []
     for kw in (dict(), dict(modulation="ASK", sample_rate=250e3, timestamp=3.0)):
-        mine, ref = Signal("", "n", **kw), ns.Signal("", "n", **kw)
-        for attr in ("name", "tolerance", "samples_per_symbol", "pause_threshold", "message_length_divisor", "costas_loop_bandwidth",
-                     "center", "sample_rate", "bits_per_symbol", "center_spacing", "modulation_type", "timestamp", "noise_threshold",
-                     "already_demodulated", "modulation_order"):
-            assert getattr(mine, attr) == getattr(ref, attr), attr
-        assert mine.parameter_cache == ref.parameter_cache
+        sig = Signal("", "n", **kw)
+        out.append([getattr(sig, attr) for attr in ("name", "tolerance", "samples_per_symbol", "pause_threshold", "message_length_divisor",
+                                                    "costas_loop_bandwidth", "center", "sample_rate", "bits_per_symbol", "center_spacing",
+                                                    "modulation_type", "timestamp", "noise_threshold", "already_demodulated",
+                                                    "modulation_order")])
+        out.append(sig.parameter_cache)
+    return out
 
 
-def test_edit_operations_match_reference():
-    """insert / delete / mute / crop (Signal.py:613-651) on host data: same samples, same cached demodulation, same flags"""
-    from oracle import ref_loader
-    ns = ref_loader.load_python_layer()
-    from urh_b200.signalprocessing.Signal import Signal
-
+def observe_edit_operations(Signal):
+    """insert / delete / mute / crop (Signal.py:613-651) on host data: samples, cached demodulation, flags"""
     rng = np.random.default_rng(8)
+    out = []
     for trial in range(20):
         n = int(rng.integers(20, 200))
         iq = rng.integers(-100, 100, (n, 2)).astype(np.int16) if trial % 2 else rng.standard_normal((n, 2)).astype(np.float32)
-        mine, ref = Signal.from_samples(iq.copy(), "e", 1e6), ns.Signal.from_samples(iq.copy(), "e", 1e6)
-        qad = rng.standard_normal(n).astype(np.float32)
-        for s in (mine, ref):
-            s._qad = qad.copy()
-            s.parameter_cache["FSK"]["center"] = 0.5
+        s = Signal.from_samples(iq.copy(), "e", 1e6)
+        s._qad = rng.standard_normal(n).astype(np.float32)
+        s.parameter_cache["FSK"]["center"] = 0.5
         a, b = sorted(int(v) for v in rng.integers(0, n, 2))
         op = trial % 4
-        for s in (mine, ref):
-            if op == 0:
-                s.mute_range(a, b)
-            elif op == 1:
-                s.delete_range(a, b)
-            elif op == 2:
-                s.crop_to_range(a, max(b, a + 1))
-            else:
-                s.insert_data(a, iq[:5].copy())
-        assert np.array_equal(mine.iq_array.data, ref.iq_array.data), (trial, op)
-        assert (mine._qad is None) == (ref._qad is None), (trial, op)
-        if mine._qad is not None:
-            assert np.array_equal(mine._qad, ref._qad), (trial, op)
-        assert mine.changed == ref.changed and mine.num_samples == ref.num_samples
-        assert mine.parameter_cache == ref.parameter_cache
+        if op == 0:
+            s.mute_range(a, b)
+        elif op == 1:
+            s.delete_range(a, b)
+        elif op == 2:
+            s.crop_to_range(a, max(b, a + 1))
+        else:
+            s.insert_data(a, iq[:5].copy())
+        out.append([s.iq_array.data, s._qad is None, s._qad, s.changed, s.num_samples, s.parameter_cache])
+    return out
+
+
+def test_parameter_setters_match_reference():
+    from urh_b200.signalprocessing.Signal import Signal
+
+    obs = observe_parameter_setters(Signal)
+    assert obs[-1] == 8
+    assert_matches_reference("signal_parameter_setters", obs)
+
+
+def test_construction_defaults_match_reference():
+    from urh_b200.signalprocessing.Signal import Signal
+
+    assert_matches_reference("signal_construction_defaults", observe_construction_defaults(Signal))
+
+
+def test_edit_operations_match_reference():
+    from urh_b200.signalprocessing.Signal import Signal
+
+    assert_matches_reference("signal_edit_operations", observe_edit_operations(Signal))
